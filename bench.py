@@ -13,6 +13,10 @@ scheduler 3k_steps_clipping_rescaling; synthetic images, seed-0 random-init weig
                                                              example config), through `_classifier_free_guidance_forward_start`
 Under torchrun (N > 1): one rank per GPU, batch-sharded (weak scaling), one final NCCL all-gather of the outputs.
 Prints ONE JSON line on rank 0.
+
+  python bench.py --dump-outputs DIR [...]                   also writes what the last timed step returned as DIR/<name>.npy
+                                                             (float32, rank 0): inputs and weights are seeded, so two builds run
+                                                             with the same arguments can be compared output for output
 """
 import argparse
 import json
@@ -31,6 +35,7 @@ if ROOT not in sys.path:
 GFLOP_PER_IMAGE_FORWARD = {("small_denoiser_config", 128): 285.58, ("small_denoiser_config", 64): 68.98,
                            ("super_small", 128): 74.67, ("super_small", 64): 17.46}   # SURVEY §8(d)
 METRIC = "images/sec, DDIM invert+regenerate 128x128 100 steps"
+DUMP_MAX_BYTES = 64 * 10**6
 
 
 def measured_traffic():
@@ -71,7 +76,36 @@ def parse():
     p.add_argument("--dump-ops", default="", help="write the per-op device-time table (sampled forwards) to this markdown file")
     p.add_argument("--cpu-sample-images", type=int, default=12)   # ~12 s of 16-thread CPU work on the GPU box (4 images took 4.2 s)
     p.add_argument("--cpu-sample-steps", type=int, default=1)
-    return p.parse_args()
+    p.add_argument("--dump-outputs", default="", metavar="DIR",
+                   help="write the arrays the last timed step returned to DIR/<name>.npy (float32, at most 64 MB in all; a larger "
+                        "array is replaced by a fixed seeded sample of its elements)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        p.error("--dump-outputs writes the outputs of the CUDA arm; the reference arm only times a sample of the workload")
+    return args
+
+
+def dump_outputs(path, arrays):
+    """Writes each named array as float32 `path/<name>.npy`.  An array larger than its share of DUMP_MAX_BYTES is replaced by
+    the elements at a fixed set of flat positions (numpy seed 0, sorted), the same positions in every run of the same shape."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    cap = (DUMP_MAX_BYTES // len(arrays) - 4096) // 4        # 4 KB per file left for the .npy header
+    for name, a in arrays.items():
+        a = np.asarray(a.detach().float().cpu() if hasattr(a, "detach") else a, dtype=np.float32)
+        if a.size > cap:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
+def pil_stack(imgs):
+    """PIL images (what the drop-in calls return) as one (B, H, W, C) array of their 0..255 values."""
+    import numpy as np
+
+    return np.stack([np.asarray(im) for im in imgs])
 
 
 def peaks():
@@ -353,11 +387,13 @@ def run_ours(args):
     e0.record()
     for _ in range(args.steps):
         flush.fill_(1)            # L2 flush between timed iterations
-        step()
+        out = step()
     e1.record()
     sync()
     ms = e0.elapsed_time(e1)
     prof = unet.profile_end()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"images": out})
     if rank == 0 and args.dump_ops:
         ops = unet.profile_ops()
         tot = sum(o["ms"] for o in ops) or 1.0
@@ -477,6 +513,8 @@ def run_cfg(args, pipe, unet, x_host, x_dev, tgt, tgt_d, dev, rank, world, local
     assert len(imgs) == args.batch
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"images": pil_stack(imgs)})
     # UNet kernels (counted by the library: the guidance combine and the scheduler update live in conv_out's epilogue on the fused
     # route, `pd_cfg_transfer`) + per call: add_noise, denorm
     launches = unet.launch_count() - l0 + args.steps * 2
@@ -553,6 +591,8 @@ def run_guided(args, pipe, unet, x_host, x_dev, src, src_d, tgt, tgt_d, dev, ran
     sync()
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"images": pil_stack(imgs)})
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -626,6 +666,8 @@ def run_train(args, pipe, unet, x_host, x_dev, labels, labels_d, dev, rank, worl
     sync()
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:      # the loss the step returned and the parameters it left (before the e2e steps move them)
+        dump_outputs(args.dump_outputs, {"loss": loss, "parameters": trainer.params})
     launches = trainer.launch_count() - l0 + args.steps * 4      # + add_noise, adamw (memset + sumsq + update)
     t = torch.tensor([ms], device=dev)
     if world > 1:

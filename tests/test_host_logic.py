@@ -243,6 +243,32 @@ def test_bench_reference_arm_other_ranks_exit_without_work():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_bench_dump_outputs_float32_within_budget_and_fixed_sample(tmp_path, monkeypatch):
+    import bench
+
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 64 << 10)
+    big = torch.arange(100_000, dtype=torch.float64)
+    small = np.arange(6, dtype=np.uint8).reshape(2, 3)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"big": big, "small": small})
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64 << 10
+    s = np.load(tmp_path / "a" / "small.npy")
+    assert s.dtype == np.float32 and s.tolist() == small.tolist()
+    a, b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert a.dtype == np.float32 and 0 < a.size < big.numel() and np.array_equal(a, b)
+    assert np.all(np.diff(a) > 0)        # distinct positions, in order
+
+
+def test_bench_rejects_zero_steps_and_dump_on_reference_arm(tmp_path):
+    import subprocess
+    import sys
+
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and out.stdout == "", (extra, out.stderr[-500:])
+    assert list(tmp_path.iterdir()) == []
+
+
 def test_cfg_lookup_reads_attribute_and_dict_configs():
     from types import SimpleNamespace as NS
 
