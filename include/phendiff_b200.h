@@ -162,11 +162,18 @@ int pd_cfg_transfer(pd_unet_t* h, float* x, const int64_t* labels, const float* 
  *      fp32 path: every operator of the backward pass as a CUDA-core kernel (validated against torch.autograd on the oracle). */
 int pd_train_create(pd_unet_t* h, int32_t batch, int32_t height, int32_t width, pd_train_t** out);
 int pd_train_destroy(pd_train_t* t);
-/* precision 0 (default): fp32 on CUDA cores, the validation path.  1: "bf16" mixed precision as accelerate runs the reference
- * (mixed_precision="bf16", train.py:57-61): convolutions (forward, dgrad, wgrad) take bf16 operands on the tcgen05 kernels with fp32
- * accumulation for every shape those kernels support, everything else (GroupNorm, attention, embeddings, loss, optimizer, master
- * weights, gradients) stays fp32.  Changes the workspace plan: call before pd_train_workspace_bytes / pd_train_bind. */
+/* precision PD_PREC_FP32 (default): fp32 on CUDA cores, the validation path.  PD_PREC_BF16: "bf16" mixed precision as accelerate runs
+ * the reference (mixed_precision="bf16", train.py:57-61): convolutions (forward, dgrad, wgrad) take bf16 operands on the tcgen05 kernels
+ * and attention its operands on mma.sync, with fp32 accumulation, for every shape those kernels support (the PHENDIFF_B200_TRAIN_TC
+ * mask selects the pieces); everything else (GroupNorm statistics, embeddings, loss, optimizer, master weights, gradients) stays fp32.
+ * PD_PREC_FP16: the same pieces with fp16 operands, as the reference's launch scripts train (accelerate --mixed_precision=fp16).  fp16
+ * gradients need a loss scale (pd_train_set_loss_scale, pd_adamw_step_scaled) to stay above fp16's subnormal range.
+ * Changes the workspace plan: call before pd_train_workspace_bytes / pd_train_bind. */
 int pd_train_set_precision(pd_train_t* t, int32_t precision);
+/* loss scale S of every following pd_train_step_grad on this handle: the backward starts from S * d(loss), so the gradients come out
+ * multiplied by S (torch GradScaler.scale(loss).backward()); loss_out stays unscaled.  scale_dev: ONE fp32 on the device, read on the
+ * stream when the step runs (typically &state->scale of a pd_grad_scaler_state_t); NULL (the default): 1. */
+int pd_train_set_loss_scale(pd_train_t* t, const float* scale_dev);
 /* convolution forward passes / weight gradients that took the tensor-core path since creation */
 int pd_train_tc_counts(pd_train_t* t, int64_t* convs, int64_t* wgrads);
 int pd_train_num_params_flat(pd_train_t* t, int64_t* numel);
@@ -199,6 +206,29 @@ int pd_guidance_lp_grad(const pd_step_coeffs_t* step, const float* x, const floa
 int pd_adamw_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, float* ema, int64_t n, float lr, float beta1,
                   float beta2, float eps, float weight_decay, int32_t step, float max_grad_norm, float ema_decay, float* scratch,
                   float* grad_norm_out, pd_stream_t stream);
+
+/* Dynamic loss scaling (torch.amp.GradScaler, what accelerate builds for mixed_precision="fp16"), kept on the device so that the training
+ * step never waits for the host.  Initialise on the host (scale = init_scale, everything else 0) and copy to the device once. */
+typedef struct pd_grad_scaler_state {
+    float scale;              /* S: the loss scale the next backward multiplies by (GradScaler._scale) */
+    int32_t growth_tracker;   /* consecutive applied steps since the last scale change (GradScaler._growth_tracker) */
+    int32_t optimizer_steps;  /* AdamW steps applied: AdamW's step count (bias correction) and what LambdaLR counts */
+    int32_t found_inf;        /* 1 when the last pass found an inf / NaN gradient and skipped the step */
+    int32_t skipped_steps;    /* passes skipped since initialisation */
+} pd_grad_scaler_state_t;
+/* pd_adamw_step on loss-scaled gradients, one optimizer step of accelerate's fp16 loop: GradScaler.unscale_ (inv = 1 / S, found_inf =
+ * any gradient inf or NaN, g *= inv), clip_grad_norm_ on the unscaled gradients, GradScaler.step (AdamW runs only when no gradient was
+ * inf / NaN: otherwise parameters and moments stay bit-identical and the AdamW step count does not advance), GradScaler.update (found_inf:
+ * S *= backoff_factor, tracker = 0; else tracker + 1, and at growth_interval S *= growth_factor if finite, tracker = 0), then the EMA
+ * step, which runs on skipped steps too (toward the unchanged parameters).  grads are read, not modified.  The bias correction uses
+ * state->optimizer_steps; lr applies to the step when it is not skipped.  scratch: PD_ADAMW_SCALED_SCRATCH_FLOATS fp32 on the device;
+ * grad_norm_out (optional): the norm of the unscaled gradients (non-finite on a skipped step).  Deterministic: data-parallel replicas
+ * with the same gradients keep bit-identical parameters and scaler state. */
+#define PD_ADAMW_SCALED_SCRATCH_FLOATS 2376
+int pd_adamw_step_scaled(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, float* ema, int64_t n, float lr,
+                         float beta1, float beta2, float eps, float weight_decay, float max_grad_norm, float ema_decay,
+                         pd_grad_scaler_state_t* state, float growth_factor, float backoff_factor, int32_t growth_interval,
+                         float* scratch, float* grad_norm_out, pd_stream_t stream);
 
 /* number of kernels launched by this handle since creation (bench.py's gpu_launches) */
 int pd_unet_launch_count(pd_unet_t* h, int64_t* n);

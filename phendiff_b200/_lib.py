@@ -37,6 +37,16 @@ class StepCoeffs(C.Structure):
     ]
 
 
+class GradScalerState(C.Structure):
+    """pd_grad_scaler_state_t: torch.amp.GradScaler's state, kept on the device by pd_adamw_step_scaled."""
+    _fields_ = [("scale", C.c_float), ("growth_tracker", C.c_int32), ("optimizer_steps", C.c_int32), ("found_inf", C.c_int32),
+                ("skipped_steps", C.c_int32)]
+
+
+PD_ADAMW_SCRATCH_FLOATS = 1185
+PD_ADAMW_SCALED_SCRATCH_FLOATS = 2376
+
+
 class TestConvArgs(C.Structure):
     """pd_test_conv_args_t (kernel-level test entry point)."""
     _fields_ = ([(n, C.c_int32) for n in ("impl", "dtype", "n", "h", "w", "c1", "c2", "cout", "ksize", "stride", "pad", "upsample",
@@ -70,6 +80,7 @@ _SIGNATURES = {
     "pd_train_create": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.POINTER(_P)]),
     "pd_train_destroy": (C.c_int, [_P]),
     "pd_train_set_precision": (C.c_int, [_P, C.c_int32]),
+    "pd_train_set_loss_scale": (C.c_int, [_P, _P]),
     "pd_train_tc_counts": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "pd_train_num_params_flat": (C.c_int, [_P, C.POINTER(C.c_int64)]),
     "pd_train_param_offset": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int64)]),
@@ -82,6 +93,8 @@ _SIGNATURES = {
     "pd_guidance_lp_grad": (C.c_int, [C.POINTER(StepCoeffs), _P, _P, _P, C.c_int32, C.c_int64, C.c_float, _P, _P, _P, _P, _P]),
     "pd_adamw_step": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_int32,
                                  C.c_float, C.c_float, _P, _P, _P]),
+    "pd_adamw_step_scaled": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
+                                        C.c_float, _P, C.c_float, C.c_float, C.c_int32, _P, _P, _P]),
     "pd_debug_pair_kernel_launches": (C.c_longlong, []),
     "pd_unet_launch_count": (C.c_int, [_P, C.POINTER(C.c_int64)]),
     "pd_unet_plan_info": (C.c_int, [_P, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),

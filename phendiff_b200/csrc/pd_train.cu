@@ -46,8 +46,10 @@ struct pd_train {
     cudaStream_t s = nullptr;
     int rc = 0;
     int64_t launches = 0;
-    // mixed precision (pd_train_set_precision): 16-bit operands for the convolutions on the tcgen05 kernels, everything else fp32
+    // mixed precision (pd_train_set_precision): 16-bit operands (bf16 or fp16) for the convolutions on the tcgen05 kernels and for
+    // attention on mma.sync, everything else fp32
     int dt = DT_F32;
+    const float* loss_scale = nullptr;   // device scalar multiplying the loss gradient (pd_train_set_loss_scale); null: 1
     unsigned tc_mask = 127;        // 1 conv forward, 2 dgrad, 4 wgrad, 8 attention, 16 16-bit-only GroupNorm outputs + fused q/k/v, 32 padded
                                    // tensor-core GEMMs for conv_in / conv_out gradients, 64 GroupNorm statistics from the conv's forward
                                    // epilogue (PHENDIFF_B200_TRAIN_TC)
@@ -599,14 +601,14 @@ struct Walk {
         float* delta = (float*)aux((size_t)B * (C / 8) * S * sizeof(float));
         if (!dry()) {
             const bool mma = t->dt != DT_F32 && (t->tc_mask & 8) && attn8_mma_supported(S, C, pitch);
-            run(mma ? launch_attn8_mma_fwd(qd, kd, vd, pitch, B, S, C, o->d, lse, s()) : launch_attn8_fwd(qd, kd, vd, pitch, B, S, C, o->d, lse, s()));
+            run(mma ? launch_attn8_mma_fwd(t->dt, qd, kd, vd, pitch, B, S, C, o->d, lse, s()) : launch_attn8_fwd(qd, kd, vd, pitch, B, S, C, o->d, lse, s()));
             count();
             const TT O = *o;
             const int Bn = B;
             pd_train* tr = t;
             bwd([=](cudaStream_t st) {
                 tr->launches += 2;
-                return mma ? launch_attn8_mma_bwd(qd, kd, vd, pitch, O.d, O.g, lse, Bn, S, C, qg, kg, vg, delta, st)
+                return mma ? launch_attn8_mma_bwd(tr->dt, qd, kd, vd, pitch, O.d, O.g, lse, Bn, S, C, qg, kg, vg, delta, st)
                            : launch_attn8_bwd(qd, kd, vd, pitch, O.d, O.g, lse, Bn, S, C, qg, kg, vg, delta, st);
             });
         }
@@ -863,8 +865,9 @@ int pd_train_create(pd_unet_t* m, int32_t batch, int32_t height, int32_t width, 
 
 int pd_train_set_precision(pd_train_t* t, int32_t precision) {
     PD_REQUIRE(t, "null argument");
-    PD_REQUIRE(precision == 0 || precision == 1, "precision: 0 = fp32 (validation path), 1 = bf16 tensor-core convolutions");
-    t->dt = precision == 1 ? DT_BF16 : DT_F32;
+    PD_REQUIRE(precision == PD_PREC_FP32 || precision == PD_PREC_BF16 || precision == PD_PREC_FP16,
+               "precision: 0 = fp32 (validation path), 1 = bf16, 2 = fp16 tensor-core operands");
+    t->dt = precision == PD_PREC_BF16 ? DT_BF16 : precision == PD_PREC_FP16 ? DT_F16 : DT_F32;
     t->ws = nullptr;   // the workspace plan changes: bind again
     float *mo, *dm;
     int rc = walk(t, true, nullptr, nullptr, nullptr, &mo, &dm);
@@ -872,6 +875,12 @@ int pd_train_set_precision(pd_train_t* t, int32_t precision) {
     t->act_bytes = t->act_bump;
     t->aux_bytes = t->aux_bump + 2 * t->scr_max + t->wstage_max;
     t->ws_bytes = 2 * t->act_bytes + t->aux_bytes + 1024;
+    return 0;
+}
+
+int pd_train_set_loss_scale(pd_train_t* t, const float* scale_dev) {
+    PD_REQUIRE(t, "null argument");
+    t->loss_scale = scale_dev;
     return 0;
 }
 
@@ -926,7 +935,7 @@ int pd_train_step_grad(pd_train_t* t, const float* params, float* grads, const f
     if (rc) return rc;
     PD_REQUIRE(t->act_bump <= t->act_bytes && t->aux_bump + 2 * t->scr_max + t->wstage_max <= t->aux_bytes, "internal: training workspace plan mismatch");
     const size_t per = (size_t)t->m->cfg.out_channels * t->H * t->W;
-    if ((rc = launch_mse_loss(mo, target, sample_weight, t->B, per, loss_out, dm, s))) return rc;
+    if ((rc = launch_mse_loss(mo, target, sample_weight, t->B, per, t->loss_scale, loss_out, dm, s))) return rc;
     if (model_out) PD_CHECK_CUDA(cudaMemcpyAsync(model_out, mo, (size_t)t->B * per * sizeof(float), cudaMemcpyDeviceToDevice, s));
     for (auto it = t->tape.rbegin(); it != t->tape.rend(); ++it)
         if ((rc = (*it)(s))) return rc;
@@ -989,6 +998,17 @@ int pd_adamw_step(float* params, const float* grads, float* exp_avg, float* exp_
     PD_REQUIRE(params && grads && exp_avg && exp_avg_sq && scratch && n > 0 && step >= 1, "bad argument");
     return launch_adamw(params, grads, exp_avg, exp_avg_sq, ema, (size_t)n, lr, beta1, beta2, eps, weight_decay, step, max_grad_norm, ema_decay,
                         scratch, grad_norm_out, (cudaStream_t)stream);
+}
+
+int pd_adamw_step_scaled(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, float* ema, int64_t n, float lr, float beta1,
+                         float beta2, float eps, float weight_decay, float max_grad_norm, float ema_decay, pd_grad_scaler_state_t* state,
+                         float growth_factor, float backoff_factor, int32_t growth_interval, float* scratch, float* grad_norm_out,
+                         pd_stream_t stream) {
+    PD_REQUIRE(params && grads && exp_avg && exp_avg_sq && state && scratch && n > 0, "bad argument");
+    PD_REQUIRE(growth_factor > 1.f && backoff_factor > 0.f && backoff_factor < 1.f && growth_interval >= 1,
+               "grad scaler: growth_factor > 1, 0 < backoff_factor < 1 and growth_interval >= 1 (torch.amp.GradScaler's conditions)");
+    return launch_adamw_scaled(params, grads, exp_avg, exp_avg_sq, ema, (size_t)n, lr, beta1, beta2, eps, weight_decay, max_grad_norm, ema_decay,
+                               state, growth_factor, backoff_factor, growth_interval, scratch, grad_norm_out, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -54,9 +54,15 @@ int launch_silu_bwd(const float* pre, const float* dact, size_t total, float* dp
 int launch_scatter_rows(const float* d, const int64_t* labels, int B, int D, float scale, float* table_grad, cudaStream_t s);
 int launch_nchw_to_nhwc_pad(const float* x, int N, int C, int HW, int Cp, float* out, cudaStream_t s);
 int launch_add_inplace(float* y, const float* x, float alpha, size_t n, cudaStream_t s);
-int launch_mse_loss(const float* m, const float* target, const float* weight, int B, size_t per, float* loss, float* dm, cudaStream_t s);
+// dm is the gradient of the loss times *loss_scale (NULL: 1); the loss itself is never scaled
+int launch_mse_loss(const float* m, const float* target, const float* weight, int B, size_t per, const float* loss_scale, float* loss, float* dm,
+                    cudaStream_t s);
 int launch_adamw(float* p, const float* g, float* m, float* v, float* ema, size_t n, float lr, float b1, float b2, float eps, float wd,
                  int step, float max_norm, float ema_decay, float* scratch_sumsq, float* norm_out, cudaStream_t s);
+// the same on loss-scaled gradients with torch.amp.GradScaler's unscale / skip-on-inf / scale update; scaler state on the device
+int launch_adamw_scaled(float* p, const float* g, float* m, float* v, float* ema, size_t n, float lr, float b1, float b2, float eps, float wd,
+                        float max_norm, float ema_decay, pd_grad_scaler_state_t* state, float growth, float backoff, int interval,
+                        float* scratch, float* norm_out, cudaStream_t s);
 
 // gradient-guided generation (f4): loss_i = || pred_original_sample(x, m) - ref ||_p per image and its gradients w.r.t. m and (directly) x
 int launch_guidance_lp_grad(const pd_step_coeffs_t& c, const float* x, const float* m, const float* ref, int B, size_t per, float p, float* sums,
@@ -78,12 +84,13 @@ int launch_relayout_tc_dgrad_s2(int dt, const float* w, int O, int I, void* out,
 int launch_colsum_cast(int dt, const float* dy, int B, int rows_per_img, int C, float* out_all, float* out_img, void* out16, cudaStream_t s);
 int launch_wgrad_unstage(const float* stage, int O, int I, int kk, float* dw, cudaStream_t s, int Opad = 0, int Ipad = 0);
 
-// softmax attention (head_dim 8) on the warp-level tensor cores, bf16 operands staged from the fp32 activations (pd_train_attn_mma.cu);
-// same interface as launch_attn8_fwd / launch_attn8_bwd
+// softmax attention (head_dim 8) on the warp-level tensor cores, 16-bit operands (dt: DT_BF16 / DT_F16) staged from the fp32 activations
+// (pd_train_attn_mma.cu); otherwise the interface of launch_attn8_fwd / launch_attn8_bwd
 bool attn8_mma_supported(int S, int C, int pitch);
-int launch_attn8_mma_fwd(const float* q, const float* k, const float* v, int pitch, int N, int S, int C, float* out, float* lse, cudaStream_t s);
-int launch_attn8_mma_bwd(const float* q, const float* k, const float* v, int pitch, const float* o, const float* dout, const float* lse, int N,
-                         int S, int C, float* dq, float* dk, float* dv, float* delta, cudaStream_t s);
+int launch_attn8_mma_fwd(int dt, const float* q, const float* k, const float* v, int pitch, int N, int S, int C, float* out, float* lse,
+                         cudaStream_t s);
+int launch_attn8_mma_bwd(int dt, const float* q, const float* k, const float* v, int pitch, const float* o, const float* dout, const float* lse,
+                         int N, int S, int C, float* dq, float* dk, float* dv, float* delta, cudaStream_t s);
 
 // tcgen05 weight gradient of a stride-1 'same' convolution (k = 1 or 3): stage[tap][co][ci] += sum_pixels dY[p, co] * X[p @ tap, ci],
 // K = pixels.  x1 / x2: the NHWC 16-bit sources of the conv input (channel concat), dy: (N, H, W, Cout) 16-bit.

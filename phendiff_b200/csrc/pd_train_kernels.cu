@@ -676,23 +676,26 @@ int launch_add_inplace(float* y, const float* x, float alpha, size_t n, cudaStre
 // loss of utils_training.py:415-433 in one form: mean over all elements of weight[b] * (m - target)^2 (epsilon: target = noise,
 // weight = 1; v_prediction: target = velocity; sample: target = clean images, weight = alpha_t / (1 - alpha_t)), and its gradient
 // ---------------------------------------------------------------------------------------------------------------------
+// dm carries the loss scale S (GradScaler.scale(loss).backward()); the loss does not.  S = 1 multiplies exactly: unscaled runs are unchanged.
 __global__ void __launch_bounds__(256) mse_loss_kernel(const float* __restrict__ m, const float* __restrict__ target,
-                                                        const float* __restrict__ weight, int B, size_t per, float* __restrict__ loss,
-                                                        float* __restrict__ dm) {
+                                                        const float* __restrict__ weight, int B, size_t per, const float* __restrict__ loss_scale,
+                                                        float* __restrict__ loss, float* __restrict__ dm) {
     const size_t total = (size_t)B * per;
     const float inv = 1.0f / (float)total;
+    const float sc = loss_scale ? *loss_scale : 1.0f;
     float acc = 0.f;
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const float w = weight ? weight[i / per] : 1.0f, d = m[i] - target[i];
         acc = fmaf(w * d, d, acc);
-        dm[i] = 2.0f * w * d * inv;
+        dm[i] = 2.0f * w * d * inv * sc;
     }
     acc = warp_sum(acc);
     if ((threadIdx.x & 31) == 0) atomicAdd(loss, acc * inv);
 }
-int launch_mse_loss(const float* m, const float* target, const float* weight, int B, size_t per, float* loss, float* dm, cudaStream_t s) {
+int launch_mse_loss(const float* m, const float* target, const float* weight, int B, size_t per, const float* loss_scale, float* loss, float* dm,
+                    cudaStream_t s) {
     PD_CHECK_CUDA(cudaMemsetAsync(loss, 0, sizeof(float), s));
-    mse_loss_kernel<<<(int)std::min<size_t>(((size_t)B * per + 255) / 256, 148 * 8), 256, 0, s>>>(m, target, weight, B, per, loss, dm);
+    mse_loss_kernel<<<(int)std::min<size_t>(((size_t)B * per + 255) / 256, 148 * 8), 256, 0, s>>>(m, target, weight, B, per, loss_scale, loss, dm);
     PD_CHECK_CUDA(cudaGetLastError());
     return 0;
 }
@@ -754,6 +757,116 @@ int launch_adamw(float* p, const float* g, float* m, float* v, float* ema, size_
     sumsq_final_kernel<<<1, 1024, 0, s>>>(scratch_sumsq, grid);
     const float bc1 = 1.0f - powf(b1, (float)step), bc2 = 1.0f - powf(b2, (float)step);
     adamw_kernel<<<grid, 256, 0, s>>>(p, g, m, v, ema, n, lr, b1, b2, eps, wd, bc1, sqrtf(bc2), max_norm, scratch_sumsq, ema_decay, norm_out);
+    PD_CHECK_CUDA(cudaGetLastError());
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// the same step on loss-scaled gradients (fp16 mixed precision): torch.amp.GradScaler unscale_ / step / update around clip + AdamW,
+// three launches like launch_adamw and just as deterministic (replicas keep bit-identical parameters AND scaler state).
+//   stage 1: per block, the sum of squares of g * inv and whether any g is inf / NaN (inv = float(1 / double(S)), GradScaler's)
+//   stage 2: one block folds both in a fixed order; one thread takes the decision: norm, clip coefficient, skip or apply, the AdamW
+//            step count and its bias corrections, the scale update.  It rewrites S, so it leaves the S the gradients were made with
+//            as inv in scratch: stage 1 has finished reading S, stage 3 reads only scratch.
+//   stage 3: AdamW on (g * inv) * coef unless skipped, then the EMA step either way.
+// scratch: [0, 8) decision (kScHdr*), [8, 8 + kSumsqBlocks) partial sums, then kSumsqBlocks non-finite flags
+// ---------------------------------------------------------------------------------------------------------------------
+enum { kScInv = 0, kScCoef = 1, kScStepSize = 2, kScBc2Sqrt = 3, kScApply = 4, kScHdr = 8 };
+static_assert(kScHdr + 2 * kSumsqBlocks == PD_ADAMW_SCALED_SCRATCH_FLOATS, "scratch layout of pd_adamw_step_scaled");
+__device__ __forceinline__ float inv_scale_of(float S) { return (float)(1.0 / (double)S); }
+__global__ void __launch_bounds__(256) sumsq_unscale_kernel(const float* __restrict__ g, size_t n, const pd_grad_scaler_state_t* __restrict__ st,
+                                                            float* __restrict__ scratch) {
+    __shared__ float red[8];
+    const float inv = inv_scale_of(st->scale);
+    float acc = 0.f;
+    bool bad = false;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const float gi = g[i];
+        bad |= !isfinite(gi);
+        const float u = gi * inv;
+        acc = fmaf(u, u, acc);
+    }
+    bad = __syncthreads_or(bad);
+    acc = warp_sum(acc);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float t = 0.f;
+        for (int w = 0; w < 8; ++w) t += red[w];
+        scratch[kScHdr + blockIdx.x] = t;
+        scratch[kScHdr + kSumsqBlocks + blockIdx.x] = bad ? 1.f : 0.f;
+    }
+}
+__global__ void __launch_bounds__(1024) scaler_decide_kernel(float* __restrict__ scratch, int nblocks, pd_grad_scaler_state_t* __restrict__ st,
+                                                             float lr, float b1, float b2, float max_norm, float growth, float backoff, int interval,
+                                                             float* __restrict__ norm_out) {
+    __shared__ double red[1024];
+    double acc = 0.0;
+    bool bad = false;
+    for (int i = threadIdx.x; i < nblocks; i += 1024) {
+        acc += (double)scratch[kScHdr + i];
+        bad |= scratch[kScHdr + kSumsqBlocks + i] != 0.f;
+    }
+    bad = __syncthreads_or(bad);
+    red[threadIdx.x] = acc;
+    __syncthreads();
+    for (int o = 512; o > 0; o >>= 1) {
+        if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+        __syncthreads();
+    }
+    if (threadIdx.x != 0) return;
+    const float S = st->scale;
+    const float norm = sqrtf((float)red[0]);
+    if (norm_out) *norm_out = norm;
+    scratch[kScInv] = inv_scale_of(S);
+    scratch[kScCoef] = max_norm > 0.f ? fminf(max_norm / (norm + 1e-6f), 1.0f) : 1.0f;
+    scratch[kScApply] = bad ? 0.f : 1.f;
+    if (bad) {                                     // GradScaler.step skips optimizer.step(); update() backs off
+        st->found_inf = 1;
+        st->skipped_steps += 1;
+        st->scale = S * backoff;
+        st->growth_tracker = 0;
+        return;
+    }
+    st->found_inf = 0;
+    const int step = ++st->optimizer_steps;
+    scratch[kScStepSize] = (float)((double)lr / (1.0 - pow((double)b1, (double)step)));
+    scratch[kScBc2Sqrt] = (float)sqrt(1.0 - pow((double)b2, (double)step));
+    const int tracker = st->growth_tracker + 1;    // torch._amp_update_scale_
+    if (tracker == interval) {
+        const float grown = S * growth;
+        if (isfinite(grown)) st->scale = grown;
+        st->growth_tracker = 0;
+    } else {
+        st->growth_tracker = tracker;
+    }
+}
+__global__ void __launch_bounds__(256) adamw_scaled_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
+                                                            float* __restrict__ v, float* __restrict__ ema, size_t n, float b1, float b2, float eps,
+                                                            float lr_wd, const float* __restrict__ scratch, float ema_decay) {
+    const bool apply = scratch[kScApply] != 0.f;
+    if (!apply && !ema) return;
+    const float inv = scratch[kScInv], coef = scratch[kScCoef], step_size = scratch[kScStepSize], bc2_sqrt = scratch[kScBc2Sqrt];
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        float pi = p[i];
+        if (apply) {
+            const float gi = (g[i] * inv) * coef;
+            pi *= 1.0f - lr_wd;
+            const float mi = b1 * m[i] + (1.0f - b1) * gi, vi = b2 * v[i] + (1.0f - b2) * gi * gi;
+            m[i] = mi; v[i] = vi;
+            pi -= step_size * mi / (sqrtf(vi) / bc2_sqrt + eps);
+            p[i] = pi;
+        }
+        if (ema) ema[i] -= (1.0f - ema_decay) * (ema[i] - pi);
+    }
+}
+int launch_adamw_scaled(float* p, const float* g, float* m, float* v, float* ema, size_t n, float lr, float b1, float b2, float eps, float wd,
+                        float max_norm, float ema_decay, pd_grad_scaler_state_t* state, float growth, float backoff, int interval,
+                        float* scratch, float* norm_out, cudaStream_t s) {
+    const int grid = (int)std::min<size_t>((n + 255) / 256, kSumsqBlocks);
+    sumsq_unscale_kernel<<<grid, 256, 0, s>>>(g, n, state, scratch);
+    scaler_decide_kernel<<<1, 1024, 0, s>>>(scratch, grid, state, lr, b1, b2, max_norm, growth, backoff, interval, norm_out);
+    adamw_scaled_kernel<<<grid, 256, 0, s>>>(p, g, m, v, ema, n, b1, b2, eps, lr * wd, scratch, ema_decay);
     PD_CHECK_CUDA(cudaGetLastError());
     return 0;
 }

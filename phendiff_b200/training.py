@@ -13,8 +13,10 @@ it keeps beside it (train.py:223-238, utils_training.py:552-556):
     optimizer / EMA           AdamW.step, lr_scheduler.step, zero_grad, EMAModel.step   (:452-454, :552-556)
 
 Everything between `noisy_images` and the updated parameters runs in the CUDA library: forward + backward of the UNet
-(`pd_train_step_grad`) and one fused clip + AdamW + EMA pass over flat vectors (`pd_adamw_step`).  Parameters, gradients and
-optimizer state are single flat fp32 tensors in parameter-table order; the module's `nn.Parameter`s are re-pointed at views of
+(`pd_train_step_grad`) and one fused clip + AdamW + EMA pass over flat vectors (`pd_adamw_step`; under fp16 mixed precision
+`pd_adamw_step_scaled`, which adds torch.amp.GradScaler's unscale / skip-on-inf / scale update with the scaler state on the
+device).  Parameters, gradients and optimizer state are single flat fp32 tensors in parameter-table order; the module's
+`nn.Parameter`s are re-pointed at views of
 the flat parameter vector (and their `.grad` at views of the flat gradient vector), so `state_dict()`, `save_pretrained` and a
 stock torch optimizer keep working on the same storage.  Under `torch.distributed` the flat gradient vector is averaged with
 ONE all-reduce (what DDP does in buckets for the reference, through accelerate).  There is no CPU fallback.
@@ -32,6 +34,12 @@ from . import _lib
 from .cond_unet_2d import CustomCondUNet2DModel
 from .schedulers import DDIMScheduler
 from .sharding import average_gradients
+
+
+# accelerate's `mixed_precision` names -> pd_train_set_precision
+PRECISIONS = {"no": _lib.PD_PREC_FP32, "bf16": _lib.PD_PREC_BF16, "fp16": _lib.PD_PREC_FP16}
+# torch.amp.GradScaler's defaults, which accelerate uses for mixed_precision="fp16" unless GradScalerKwargs are given
+GRAD_SCALER_DEFAULTS = {"init_scale": 2.0 ** 16, "growth_factor": 2.0, "backoff_factor": 0.5, "growth_interval": 2000}
 
 
 def ema_decay_at(optimization_step: int, max_decay: float = 0.9999, min_decay: float = 0.0, update_after_step: int = 0,
@@ -64,13 +72,33 @@ class DenoiserTrainer:
 
     `trainer.step(clean_images, class_labels)` is one iteration of the reference's epoch loop body; the pieces
     (`diffusion_and_backward`, `all_reduce_gradients`, `optimizer_step`) can be called separately (gradient accumulation:
-    call the first several times before the other two — gradients accumulate until `zero_grad`)."""
+    call the first several times before the other two — gradients accumulate until `zero_grad`).
+
+    `mixed_precision` takes accelerate's names: "no" (fp32 on CUDA cores, the validation path), "bf16" or "fp16" (16-bit operands on
+    the tensor cores, fp32 everything else).  "fp16" also scales the loss as accelerate's GradScaler does (`grad_scaler_kwargs`: the
+    keys of GRAD_SCALER_DEFAULTS, as in accelerate's GradScalerKwargs): a step whose gradients hold an inf or NaN is skipped and the
+    scale backs off.  `global_step` counts every step; `optimizer_steps` only the applied ones, which is what `lr_lambda` receives
+    (accelerate's scheduler does not step when the optimizer step was skipped)."""
 
     def __init__(self, denoiser_model: CustomCondUNet2DModel, noise_scheduler: DDIMScheduler, batch_size: int, resolution: int,
                  learning_rate: float = 1e-4, adam_beta1: float = 0.95, adam_beta2: float = 0.999, adam_weight_decay: float = 1e-6,
                  adam_epsilon: float = 1e-8, max_grad_norm: float = 1.0, use_ema: bool = False, ema_max_decay: float = 0.9999,
                  ema_inv_gamma: float = 1.0, ema_power: float = 0.75, lr_lambda: Optional[Callable[[int], float]] = None,
-                 proba_uncond: float = 0.0, mixed_precision: str = "no", shared_seed: int = 0):
+                 proba_uncond: float = 0.0, mixed_precision: str = "no", shared_seed: int = 0, grad_scaler_kwargs: Optional[dict] = None):
+        if mixed_precision not in PRECISIONS:
+            raise ValueError(f"mixed_precision must be 'no', 'bf16' or 'fp16' (accelerate's names), not {mixed_precision!r}")
+        scaler = None
+        if mixed_precision == "fp16":
+            unknown = set(grad_scaler_kwargs or {}) - set(GRAD_SCALER_DEFAULTS)
+            if unknown:
+                raise ValueError(f"grad_scaler_kwargs: unknown keys {sorted(unknown)}; accepted: {sorted(GRAD_SCALER_DEFAULTS)}")
+            scaler = dict(GRAD_SCALER_DEFAULTS, **(grad_scaler_kwargs or {}))
+            if not (scaler["init_scale"] > 0 and scaler["growth_factor"] > 1.0 and 0.0 < scaler["backoff_factor"] < 1.0
+                    and int(scaler["growth_interval"]) >= 1):
+                raise ValueError(f"grad_scaler_kwargs: need init_scale > 0, growth_factor > 1, 0 < backoff_factor < 1, growth_interval >= 1; "
+                                 f"got {scaler}")
+        elif grad_scaler_kwargs is not None:
+            raise ValueError("grad_scaler_kwargs applies to mixed_precision='fp16' only")
         self.model = denoiser_model
         self.noise_scheduler = noise_scheduler
         self.batch_size, self.resolution = int(batch_size), int(resolution)
@@ -92,11 +120,9 @@ class DenoiserTrainer:
             t = C.c_void_p()
             _lib.check(L.pd_train_create(h, self.batch_size, self.resolution, self.resolution, C.byref(t)))
             self._t, self._h = t, h
-            if mixed_precision not in ("no", "bf16"):
-                raise ValueError(f"mixed_precision must be 'no' or 'bf16' (accelerate's names), not {mixed_precision!r}")
             self.mixed_precision = mixed_precision
-            if mixed_precision == "bf16":
-                _lib.check(L.pd_train_set_precision(t, 1))
+            if mixed_precision != "no":
+                _lib.check(L.pd_train_set_precision(t, PRECISIONS[mixed_precision]))
             n = C.c_int64()
             _lib.check(L.pd_train_num_params_flat(t, C.byref(n)))
             self.numel = n.value
@@ -126,8 +152,20 @@ class DenoiserTrainer:
             self._ws_ptr = (base + 255) // 256 * 256
             _lib.check(L.pd_train_bind(t, C.c_void_p(self._ws_ptr), ws.value))
             self._loss = torch.zeros(1, device=dev, dtype=torch.float32)
-            self._scratch = torch.zeros(1185, device=dev, dtype=torch.float32)      # PD_ADAMW_SCRATCH_FLOATS
             self.grad_norm = torch.zeros(1, device=dev, dtype=torch.float32)
+            self._scaler = scaler
+            if scaler is None:
+                self._scratch = torch.zeros(_lib.PD_ADAMW_SCRATCH_FLOATS, device=dev, dtype=torch.float32)
+            else:
+                self._scratch = torch.zeros(_lib.PD_ADAMW_SCALED_SCRATCH_FLOATS, device=dev, dtype=torch.float32)
+                st = _lib.GradScalerState(scale=float(scaler["init_scale"]))
+                self._scaler_state = torch.frombuffer(bytearray(bytes(st)), dtype=torch.uint8).to(dev)
+                # the state as the last optimizer pass left it, copied back without a host wait (read once `_scaler_event` completed)
+                self._scaler_host = torch.empty(C.sizeof(_lib.GradScalerState), dtype=torch.uint8, pin_memory=True)
+                self._scaler_host.copy_(self._scaler_state.cpu())
+                self._scaler_event = None
+                # GradScalerState.scale is at offset 0: every backward of this handle multiplies the loss gradient by the current S
+                _lib.check(L.pd_train_set_loss_scale(t, C.c_void_p(self._scaler_state.data_ptr())))
             self._acp = noise_scheduler.alphas_cumprod.to(device=dev, dtype=torch.float32)
         denoiser_model.mark_dirty()     # the inference handle re-reads the (moved) parameters on its next use
 
@@ -142,6 +180,9 @@ class DenoiserTrainer:
 
     # ------------------------------------------------------------------------------------------------------------
     def named_gradients(self):
+        """(name, gradient view) per parameter.  Under mixed_precision="fp16" the gradients between the backward and `optimizer_step`
+        are the SCALED ones (loss scale `get_scale()` times the true gradient), as `param.grad` holds them under torch's GradScaler
+        before `unscale_`."""
         for name, (off, cnt, shape) in self._views.items():
             yield name, self.grads[off: off + cnt].view(shape)
 
@@ -236,21 +277,61 @@ class DenoiserTrainer:
         """Average the flat gradient vector over the data-parallel ranks: one collective (NCCL over NVLink on the GPU box)."""
         average_gradients(self.grads, group)
 
+    # ---- dynamic loss scaling (mixed_precision="fp16") ---------------------------------------------------------------------
+    def scaler_state(self) -> Optional[dict]:
+        """The device-resident GradScaler state as the last optimizer pass left it (waits for that pass), or None outside fp16 mode:
+        scale, growth_tracker, optimizer_steps (applied), found_inf (of the last step), skipped_steps."""
+        if self._scaler is None:
+            return None
+        if self._scaler_event is not None:
+            self._scaler_event.synchronize()
+        st = _lib.GradScalerState.from_buffer_copy(self._scaler_host.numpy().tobytes())
+        return {name: getattr(st, name) for name, _ in _lib.GradScalerState._fields_}
+
+    def get_scale(self) -> float:
+        """GradScaler.get_scale(): the loss scale the next backward uses (1.0 when no scaling is active).  Synchronises."""
+        return float(self.scaler_state()["scale"]) if self._scaler is not None else 1.0
+
+    @property
+    def step_was_skipped(self) -> bool:
+        """Whether the last optimizer step was skipped for inf / NaN gradients (accelerate's `optimizer.step_was_skipped`).  Synchronises."""
+        return bool(self.scaler_state()["found_inf"]) if self._scaler is not None else False
+
+    @property
+    def optimizer_steps(self) -> int:
+        """AdamW steps applied: `global_step` minus the skipped ones (fp16 mode: waits for the last optimizer pass)."""
+        return self.scaler_state()["optimizer_steps"] if self._scaler is not None else self.global_step
+
     def current_lr(self) -> float:
-        return self.lr * (self.lr_lambda(self.global_step) if self.lr_lambda is not None else 1.0)
+        return self.lr * (self.lr_lambda(self.optimizer_steps) if self.lr_lambda is not None else 1.0)
 
     def optimizer_step(self):
-        """clip_grad_norm_(1.0) + AdamW.step + lr_scheduler.step + zero_grad + EMAModel.step, one pass over the flat vectors."""
+        """clip_grad_norm_(1.0) + AdamW.step + lr_scheduler.step + zero_grad + EMAModel.step, one pass over the flat vectors.  fp16 mode:
+        GradScaler.unscale_ / step / update around them, decided on the device; the host does not wait for the outcome (it only waits
+        for the previous step's pass when `lr_lambda` needs the applied-step count)."""
         step = self.global_step + 1
         decay = 0.0
         if self.use_ema:
             decay = ema_decay_at(step, max_decay=self.ema_max_decay, inv_gamma=self.ema_inv_gamma, power=self.ema_power)
             self.cur_decay_value = decay
         with torch.cuda.device(self.device):
-            _lib.check(_lib.lib().pd_adamw_step(_lib.ptr(self.params), _lib.ptr(self.grads), _lib.ptr(self.exp_avg), _lib.ptr(self.exp_avg_sq),
-                                               _lib.ptr(self.ema), self.numel, self.current_lr(), self.betas[0], self.betas[1], self.eps,
-                                               self.weight_decay, step, self.max_grad_norm, decay, _lib.ptr(self._scratch),
-                                               _lib.ptr(self.grad_norm), _lib.current_stream()))
+            L, stream = _lib.lib(), _lib.current_stream()
+            if self._scaler is None:
+                _lib.check(L.pd_adamw_step(_lib.ptr(self.params), _lib.ptr(self.grads), _lib.ptr(self.exp_avg), _lib.ptr(self.exp_avg_sq),
+                                           _lib.ptr(self.ema), self.numel, self.current_lr(), self.betas[0], self.betas[1], self.eps,
+                                           self.weight_decay, step, self.max_grad_norm, decay, _lib.ptr(self._scratch),
+                                           _lib.ptr(self.grad_norm), stream))
+            else:
+                sc = self._scaler
+                _lib.check(L.pd_adamw_step_scaled(_lib.ptr(self.params), _lib.ptr(self.grads), _lib.ptr(self.exp_avg), _lib.ptr(self.exp_avg_sq),
+                                                  _lib.ptr(self.ema), self.numel, self.current_lr(), self.betas[0], self.betas[1], self.eps,
+                                                  self.weight_decay, self.max_grad_norm, decay, C.c_void_p(self._scaler_state.data_ptr()),
+                                                  sc["growth_factor"], sc["backoff_factor"], int(sc["growth_interval"]),
+                                                  _lib.ptr(self._scratch), _lib.ptr(self.grad_norm), stream))
+                self._scaler_host.copy_(self._scaler_state, non_blocking=True)
+                if self._scaler_event is None:
+                    self._scaler_event = torch.cuda.Event()
+                self._scaler_event.record()
         self.global_step = step
         self.zero_grad()
         self.model.mark_dirty()

@@ -110,7 +110,8 @@ def _classifier_free_guidance_forward_start(pipe: ConditionalDDIMPipeline, clean
 # ---------------------------------------------------------------------------------------------------------------------
 def _guidance_engine(pipe: ConditionalDDIMPipeline, batch: int, resolution: int, mixed_precision: Optional[str] = None):
     """The forward + input-gradient engine of the UNet for this batch shape (workspace of the training walk), cached on the pipeline.
-    mixed_precision: "bf16" (tensor-core convolutions) or "no" (fp32 validation path); default: "no" for an fp32 model, else "bf16"."""
+    mixed_precision: "bf16" or "fp16" (16-bit tensor-core operands; fp16 is the reference's autocast type for class transfer) or "no"
+    (fp32 validation path); default: "no" for an fp32 model, else "bf16".  The input gradient is not loss-scaled, as in the reference."""
     from .training import DenoiserTrainer
 
     if mixed_precision is None:

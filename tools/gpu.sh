@@ -11,7 +11,9 @@
 #   bench[:<args>]        bench.py (default workload) -> bench_<tag>.json + per-op table
 #   cfg                   bench.py --workload cfg
 #   train[:<args>]        bench.py --workload train (SURVEY f2: one training step, batch 64/GPU);  trainlaunches[:batch]: its ncu launch list by kernel
-#   ddpcheck              2-GPU NCCL check of the data-parallel training step (all-reduced gradient = mean of shard gradients; identical parameters)
+#   ddpcheck[:fp16]       2-GPU NCCL check of the data-parallel training step (all-reduced gradient = mean of shard gradients; identical parameters);
+#                         fp16: under dynamic loss scaling, plus a step that overflows on one rank only and must be skipped on every rank
+#   trainprec[:<args>]    tools/bench_train_precision.py: bf16 vs fp16 training step alternated in one process (batch 64, 128x128)
 #   guided                bench.py --workload guided (SURVEY f4: inversion + gradient-guided generation, batch 64)
 #   train2                the same at 2 GPUs (torchrun; run under `gpurun --gpus 2`)
 #   strong                strong-scaling line: total batch 256 over --gpus N ranks is not applicable at N=1; runs --batch 32 (the per-GPU share of 8)
@@ -86,8 +88,10 @@ PY
           --workload train --batch 64 --steps 3 --warmup 3 --no-cpu-baseline > gpurun_out/bench_train_n${arg:-8}_${tag}.json 2> gpurun_out/bench_train_n${arg:-8}_${tag}.err; echo "trainN exit=$?"
       tail -c 600 gpurun_out/bench_train_n${arg:-8}_${tag}.json; tail -2 gpurun_out/bench_train_n${arg:-8}_${tag}.err;;
     ddpcheck)  # needs `gpurun --gpus 2`
-      timeout 300 python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29513 tools/check_ddp_train.py \
+      timeout 300 python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29513 tools/check_ddp_train.py ${arg:+--precision $arg} \
           > gpurun_out/ddpcheck_${tag}.log 2>&1; echo "ddpcheck exit=$?"; grep ddpcheck gpurun_out/ddpcheck_${tag}.log;;
+    trainprec)   # JSON lines on stdout
+      timeout 900 python tools/bench_train_precision.py $arg; echo "trainprec exit=$?";;
     strong)
       python bench.py --batch 32 --steps 3 --warmup 3 --no-cpu-baseline > gpurun_out/bench_strong32_${tag}.json 2> gpurun_out/bench_strong32_${tag}.err; echo "strong exit=$?"; tail -c 1200 gpurun_out/bench_strong32_${tag}.json;;
     launches)
